@@ -11,7 +11,7 @@ wheel, same inputs, same box):
     cfg4  deform_conv2d 3x3, N=32 C=512->512 64x64, bf16 (tcgen05 path)                      TFLOP/s
     cfg5  resize        bilinear antialias, 128 x 3x2160x3840 fp16 -> 224x224 per rank       images/s
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--configs 2,3,4,5]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--configs 2,3,4,5] [--dump-outputs DIR]
   torchrun --nproc-per-node N ... bench.py --gpus N ...      (one rank per GPU, NCCL)
 
 N > 1 is weak scaling: every rank owns its own images.  Images are independent units, so the timed step has NO
@@ -22,6 +22,12 @@ pinned host memory (the e2e leg moves ~100 MB per step per rank through the host
 
 Timing: W >= 3 warm-up steps; L2 is flushed (256 MiB write) before every timed step; each step is bracketed by CUDA
 events on the launching stream and the K step times are summed; barrier + synchronize on both sides; max over ranks.
+Every timed loop of this project's path (headline, configs, e2e, all-gather legs) runs K steps; the legs that time the
+reference keep their own small sample sizes.
+`--dump-outputs DIR` writes, on rank 0, what the last timed step of each measured op returned as DIR/<name>.npy: the
+headline roi_align output in full, and of the configs' larger outputs a fixed sample of DUMP_SAMPLE elements at seeded
+positions (float32; integer results as float64).  The inputs are seeded, so two builds run with the same arguments can
+be compared output for output.
 `--impl reference` times the reference's own CPU kernel of the headline op (installed torchvision wheel; the oracle port
 if it is absent) on the host cores.
 """
@@ -56,6 +62,8 @@ CFG3_BOXES = 100_000
 CFG4_FLOPS = 2 * 32 * 64 * 64 * 512 * 512 * 9          # SURVEY.md §8d cfg4: 618,475,290,624
 CFG5_BATCH = 128
 CFG5_BYTES_PER_IMAGE = 3 * 2160 * 3840 * 2 + 3 * 224 * 224 * 2
+DUMP_SAMPLE = 1 << 20            # elements kept of a config output larger than this (--dump-outputs)
+DUMP_LIMIT = 64 << 20            # bytes written by --dump-outputs in all: 50.2 MB headline + <= 3.2 MB cfg3 + 2 x 4.2 MB samples
 
 
 def _peaks_json() -> dict:
@@ -208,8 +216,10 @@ def run_reference(args, rank: int):
         fn()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        fn()
+        out = fn()
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, {"cfg2_roi_align": host_array(torch.as_tensor(out))})
     ms = dt / args.steps * 1e3
     val = K_ROIS / (ms / 1e3)
     line = {
@@ -228,10 +238,42 @@ def run_reference(args, rank: int):
 # ------------------------------------------------------------------------------------------------------------------
 # measurement helpers (product arm)
 # ------------------------------------------------------------------------------------------------------------------
+def host_array(t, sample=None):
+    """`t` on the host as float32 (integer results as float64, which holds them exactly).  With `sample`, an output of more
+    elements keeps only `sample` of them, flattened, at positions drawn from a fixed seed: the same positions in every run."""
+    import numpy as np
+    import torch
+
+    t = t.detach()
+    if sample is not None and t.numel() > sample:
+        pos = np.sort(np.random.default_rng(0).choice(t.numel(), sample, replace=False))
+        t = t.reshape(-1)[torch.from_numpy(pos).to(t.device)]
+    t = t.cpu()
+    return (t.float() if t.is_floating_point() else t.double()).numpy()
+
+
+def write_outputs(path: str, arrays: dict) -> None:
+    import numpy as np
+
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 class Ctx:
     def __init__(self, torch, dist, dev, rank, world, args):
         self.torch, self.dist, self.dev, self.rank, self.world, self.args = torch, dist, dev, rank, world, args
         self.flush = torch.empty(256 * 1024 * 1024, dtype=torch.uint8, device=dev)
+        self.last = None                                      # what the last timed step of device_ms returned
+        self.outputs = {} if args.dump_outputs and rank == 0 else None
+
+    def keep_output(self, name: str, t, sample=None):
+        """Keeps a host copy of `t` for --dump-outputs (rank 0 only)."""
+        if self.outputs is not None:
+            self.outputs[name] = host_array(t, sample)
 
     def barrier(self):
         self.torch.cuda.synchronize()
@@ -260,8 +302,9 @@ class Ctx:
         for i in range(steps):
             if flush:
                 self.flush.zero_()
+            self.last = None                  # the previous step's output is freed before this step, as when nothing keeps it
             starts[i].record(stream)
-            fn()
+            self.last = fn()
             ends[i].record(stream)
         self.barrier()
         return self.max_over_ranks(sum(s.elapsed_time(e) for s, e in zip(starts, ends)) / steps)
@@ -334,19 +377,23 @@ def block_cfg3(ctx: Ctx, vb, tv, sharded) -> dict:
 
     imgs = [workloads.cfg3_batched_nms(seed=ctx.rank * CFG3_IMAGES + j) for j in range(CFG3_IMAGES)]
     dimgs = [tuple(t.to(ctx.dev) for t in im) for im in imgs]
-    steps = max(20, min(ctx.args.steps, 50))
+    steps = ctx.args.steps
     kept = [0]
 
     def step():
-        kept[0] = sum(int(tv.ops.batched_nms(b, s, i, 0.5).numel()) for (b, s, i) in dimgs)
+        keep = [tv.ops.batched_nms(b, s, i, 0.5) for (b, s, i) in dimgs]
+        kept[0] = sum(int(k.numel()) for k in keep)
+        return keep
 
     ms = ctx.device_ms(step, steps)
+    for j, k in enumerate(ctx.last):
+        ctx.keep_output(f"cfg3_batched_nms_keep_image{j}", k)
     boxes = ctx.world * CFG3_IMAGES * CFG3_BOXES
     alg = CFG3_IMAGES * (CFG3_BOXES * (16 + 4 + 8)) + 8 * kept[0]
     peak, src = peaks()
     cl = workloads.cfg3_batched_nms(seed=1000 + ctx.rank, clustered=True)
     cld = tuple(t.to(ctx.dev) for t in cl)
-    ms_cl = ctx.device_ms(lambda: tv.ops.batched_nms(*cld, 0.5), 10)
+    ms_cl = ctx.device_ms(lambda: tv.ops.batched_nms(*cld, 0.5), steps)
     out = {
         "metric": "batched_nms boxes/s", "value": boxes / (ms / 1e3), "unit": "boxes/s", "ms_per_step": ms, "steps": steps, "dtype": "f32",
         "config": {"workload": f"batched_nms fp32, {CFG3_BOXES} boxes x 80 classes per image (uniform boxes, distinct scores), "
@@ -363,7 +410,7 @@ def block_cfg3(ctx: Ctx, vb, tv, sharded) -> dict:
     }
     # e2e: one image per step
     b, s, i = imgs[0]
-    ems, h2d, d2h = ctx.e2e_ms([b, s, i], lambda bb, ss, ii: tv.ops.batched_nms(bb, ss, ii, 0.5), (CFG3_BOXES, torch.int64), 10)
+    ems, h2d, d2h = ctx.e2e_ms([b, s, i], lambda bb, ss, ii: tv.ops.batched_nms(bb, ss, ii, 0.5), (CFG3_BOXES, torch.int64), steps)
     out["e2e"] = {"value": ctx.world * CFG3_BOXES / (ems / 1e3), "unit": "boxes/s", "ms_per_step": ems, "h2d_bytes_per_step": h2d,
                   "d2h_bytes_per_step": d2h, "note": "one image per step: pinned host -> H2D -> batched_nms -> D2H of the kept indices"}
     if ctx.world > 1:
@@ -393,9 +440,10 @@ def block_cfg4(ctx: Ctx, vb, tv, sharded) -> dict:
     from vision_b200 import workloads
 
     x, off, w, b, m = workloads.cfg4_deform_conv2d(device=ctx.dev, seed=ctx.rank)
-    steps = max(20, min(ctx.args.steps, 50))
+    steps = ctx.args.steps
     op = lambda: tv.ops.deform_conv2d(x, off, w, b, 1, 1, 1, m)
     ms = ctx.device_ms(op, steps)
+    ctx.keep_output("cfg4_deform_conv2d_sample", ctx.last, DUMP_SAMPLE)
     tf = CFG4_FLOPS / (ms / 1e3) / 1e12
     burst, sustained, src = tensor_peaks()
     out = {
@@ -410,7 +458,7 @@ def block_cfg4(ctx: Ctx, vb, tv, sharded) -> dict:
     }
     hx, hoff, hw_, hb, hm = [t.cpu() for t in (x, off, w, b, m)]
     ems, h2d, d2h = ctx.e2e_ms([hx, hoff, hw_, hb, hm], lambda a, o, ww, bb, mm: tv.ops.deform_conv2d(a, o, ww, bb, 1, 1, 1, mm),
-                               (x.numel(), torch.bfloat16), 8)
+                               (x.numel(), torch.bfloat16), steps)
     out["e2e"] = {"value": ctx.world * CFG4_FLOPS / (ems / 1e3) / 1e12, "unit": "TFLOP/s", "ms_per_step": ems, "h2d_bytes_per_step": h2d,
                   "d2h_bytes_per_step": d2h}
     if ctx.world > 1:
@@ -473,8 +521,9 @@ def block_cfg5(ctx: Ctx, vb, tv, sharded) -> dict:
     from vision_b200 import workloads
 
     x = workloads.cfg5_resize(device=ctx.dev, batch=CFG5_BATCH, seed=ctx.rank)
-    steps = max(20, min(ctx.args.steps, 50))
+    steps = ctx.args.steps
     ms = ctx.device_ms(lambda: TF.resize(x, [224, 224]), steps)
+    ctx.keep_output("cfg5_resize_sample", ctx.last, DUMP_SAMPLE)
     nbytes = CFG5_BATCH * CFG5_BYTES_PER_IMAGE
     peak, src = peaks()
     out = {
@@ -489,7 +538,7 @@ def block_cfg5(ctx: Ctx, vb, tv, sharded) -> dict:
     }
     sub = 32
     hx = x[:sub].cpu()
-    ems, h2d, d2h = ctx.e2e_ms([hx], lambda a: TF.resize(a, [224, 224]), (sub * 3 * 224 * 224, torch.float16), 6)
+    ems, h2d, d2h = ctx.e2e_ms([hx], lambda a: TF.resize(a, [224, 224]), (sub * 3 * 224 * 224, torch.float16), steps)
     out["e2e"] = {"value": ctx.world * sub / (ems / 1e3), "unit": "images/s", "ms_per_step": ems, "h2d_bytes_per_step": h2d,
                   "d2h_bytes_per_step": d2h, "note": f"{sub} images per step (1.6 GB of pinned host memory), H2D-bound"}
     del hx
@@ -530,7 +579,7 @@ def block_cfg5(ctx: Ctx, vb, tv, sharded) -> dict:
                                         "its fp32 temporary is 2x the input)"}
         rows = {}
         for name, kw in (("bicubic_antialias", dict(interpolation=TF.InterpolationMode.BICUBIC)), ("bilinear_no_antialias", dict(antialias=False))):
-            o = ctx.device_ms(lambda: TF.resize(xs, [224, 224], **kw), 5)
+            o = ctx.device_ms(lambda: TF.resize(xs, [224, 224], **kw), steps)
             r = gpu_reference_ms(ctx, vb, lambda: TF.resize(xs, [224, 224], **kw), 2, 1)
             rows[name] = {"ms_per_32_images": o, "reference_ms_per_32_images": r, "ours_over_reference": r / o}
         out["secondary_modes"] = rows
@@ -547,13 +596,16 @@ def block_cfg5(ctx: Ctx, vb, tv, sharded) -> dict:
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, default=50, help="timed steps of every measurement of this project's path")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-secondary", action="store_true", help="headline (cfg2) only")
     ap.add_argument("--configs", default="2,3,4,5", help="which BASELINE configs to measure (2 is always measured)")
     ap.add_argument("--cpu-calls", type=int, default=10, help="CPU-baseline sample size (full-size calls)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step of each measured op returned as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -604,17 +656,19 @@ def main():
     wall0 = time.perf_counter()
     for i in range(args.steps):
         flush.zero_()                       # L2 flush between timed iterations (not timed)
+        out = None                          # the previous step's output is freed before this step, as when nothing keeps it
         starts[i].record(stream)
-        step()
+        out = step()
         ends[i].record(stream)
     ctx.barrier()
     wall = time.perf_counter() - wall0
     launches = vb.launch_count() - launches0
+    ctx.keep_output("cfg2_roi_align", out)
+    del out
     ms_per_step = ctx.max_over_ranks(sum(s.elapsed_time(e) for s, e in zip(starts, ends))) / args.steps
 
     # ---- end to end: pinned host buffers; EVERY step copies its inputs H2D and its result D2H ----
-    e_steps = max(6, min(args.steps, 20))
-    e2e_ms, h2d, d2h = ctx.e2e_ms([x, rois], lambda a, r: torchvision.ops.roi_align(a, r, **kw), (K_ROIS * 256 * 49, torch.float32), e_steps)
+    e2e_ms, h2d, d2h = ctx.e2e_ms([x, rois], lambda a, r: torchvision.ops.roi_align(a, r, **kw), (K_ROIS * 256 * 49, torch.float32), args.steps)
 
     # ---- the all-gather of per-shard outputs (N > 1), hidden behind the kernel ----
     # The op is cut along CHANNELS (4 x 64 planes: each chunk's input slice is contiguous for one image, and a plane-resident
@@ -627,7 +681,7 @@ def main():
         cper = xd.shape[1] // chunks
         xchunks = [xd[:, i * cper:(i + 1) * cper] for i in range(chunks)]
         assert all(c.is_contiguous() for c in xchunks)
-        g_steps = max(5, min(args.steps, 20))
+        g_steps = args.steps
         gms = ctx.device_ms(lambda: og.run(lambda i: torchvision.ops.roi_align(xchunks[i], rd, **kw), chunks), g_steps)
         plain = ctx.device_ms(lambda: sharded.all_gather_equal(torchvision.ops.roi_align(xd, rd, **kw)), g_steps)
         best = min(gms, plain)
@@ -725,6 +779,8 @@ def main():
             line["with_allgather"] = gather
         if configs:
             line["configs"] = configs
+        if ctx.outputs is not None:
+            write_outputs(args.dump_outputs, ctx.outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()

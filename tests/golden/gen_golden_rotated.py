@@ -31,10 +31,15 @@ def main():
     # test/test_ops.py-style unit boxes
     u1 = np.array([[0.5, 0.5, 1, 1, 0], [0.5, 0.5, 1, 1, 45], [0, 0, 2, 1, 30]], np.float32)
     u2 = np.array([[0.5, 0.5, 1, 1, 0], [1.0, 0.5, 1, 1, 0], [0.5, 0.5, 1, 1, 90], [0, 0, 1, 2, -60]], np.float32)
+    # the seeded boxes of tests/test_oracle.py::test_box_iou_rotated_golden_and_ref against themselves in reverse order
+    rng = np.random.default_rng(7)
+    c = rng.uniform(0, 100, (150, 2)); wh = np.exp(rng.uniform(0, 4, (150, 2))); a = rng.uniform(-360, 360, (150, 1))
+    rb = np.concatenate([c, wh, a], 1).astype(np.float32)
     ref = oracle.box_iou_rotated_ref(b1, b2)
     assert ref is not None, "oracle/_ref/libbox_iou_rotated_ref.so is missing (needs /root/reference)"
     np.savez_compressed(os.path.join(ROOT, "tests", "golden", "box_iou_rotated.npz"), boxes1=b1, boxes2=b2, ious=ref, unit1=u1,
-                        unit2=u2, unit_ious=oracle.box_iou_rotated_ref(u1, u2))
+                        unit2=u2, unit_ious=oracle.box_iou_rotated_ref(u1, u2), rand_boxes=rb,
+                        rand_ious=oracle.box_iou_rotated_ref(rb, rb[::-1].copy()))
     print("wrote box_iou_rotated.npz", ref.shape, float(ref.max()), float((ref > 0).mean()))
 
 
