@@ -507,7 +507,7 @@ def test_deform_conv2d_cfg4_reduced_vs_oracle(vb, oracle, dtype, tol):
 
     x, off, w, b, m = workloads.cfg4_deform_conv2d(batch=2, c_in=64, c_out=128, hw=32, dtype=dtype)
     if dtype != torch.float32:
-        # one accumulator (BN 128/256, 3 stages) and two accumulators (BN 512, 2 stages) of the tcgen05 kernel
+        # one accumulator (BN 128/256, 3 stages) and two accumulators (BN 512, 4 stages) of the tcgen05 kernel
         for c_out, hw in ((256, 16), (512, 12)):
             x2, off2, w2, b2, m2 = workloads.cfg4_deform_conv2d(seed=c_out, batch=1, c_in=128, c_out=c_out, hw=hw, dtype=dtype)
             want2 = oracle.deform_conv2d(x2.float().numpy(), off2.float().numpy(), w2.float().numpy(), b2.float().numpy(),

@@ -180,7 +180,7 @@ template <> struct Elem<__half> {
 struct __align__(16) TcEnt { int o[4]; float w[4]; };   // clamped corner pixel indices (y*W+x) + bilinear weights x mask
 
 // BN = output channels per CTA: 128 / 256 (one accumulator, 3 stages) or 512 (two 256-column
-// accumulators = all of TMEM, 2 stages; the A tile is then gathered once per pixel tile).
+// accumulators = all of TMEM, K depth 32, 4 stages (3 by override); the A tile is then gathered once per pixel tile).
 template <typename T, int BN, int TC_STAGES, int KB>
 __global__ void __launch_bounds__(TC1_THREADS, 1)
 deform_conv2d_tc_kernel(const T* __restrict__ nhwc, const T* __restrict__ wpacked, const T* __restrict__ offset,
@@ -993,13 +993,16 @@ bool tc2_enabled(const DcnParams& p) {
 // stage leaves room for only 2 stages, which exposes the L2 latency of every refill).
 constexpr int tc_kb(int BN) { return BN > 256 ? 32 : 64; }
 // pipeline depth: BN <= 256 -> 3 x (16 + BN/8) KB; BN = 512 -> N x 40 KB, N = 4 by default
-// (VB200_DCN_STAGES=2|3|4 overrides, for profiling: fewer stages leave more of the 228 KB to L1 — measured:
+// (VB200_DCN_STAGES=3|4 overrides, for profiling: fewer stages leave more of the 228 KB to L1 — measured:
 // no gain, profiles/deform_conv2d_r1.md).
+// No 2-stage variant: a 64-channel gather step fills both K-32 stages, so each gather group would wait on stages whose
+// previous round belongs to the other group and its own round before that; when its own previous step is still
+// unconsumed, the empty barrier is two phases behind and its parity reads as "free" - the step overwrites live operands.
 int tc_stages(int BN) {
   if (BN <= 256) return 3;
   const char* env = env_override(ENV_DCN_STAGES);
   const int n = env ? atoi(env) : 4;        // 4: each gather group owns its own pair of K-32 stages
-  return n == 2 || n == 3 ? n : 4;
+  return n == 3 ? 3 : 4;
 }
 size_t tc_smem_bytes(int BN, int KK) {
   return (size_t)tc_stages(BN) * (TC_BM + BN) * 2 * tc_kb(BN) + 128 + (size_t)KK * TC_BM * sizeof(TcEnt) + 1024;
@@ -1103,7 +1106,7 @@ int launch_tc(const void* input, const void* weight, const void* offset, const v
   }
   const int nst = tc_stages(BN);
   if (BN == 512) {
-    if (nst == 2) VB200_TC_LAUNCH(512, 2) else if (nst == 4) VB200_TC_LAUNCH(512, 4) else VB200_TC_LAUNCH(512, 3)
+    if (nst == 4) VB200_TC_LAUNCH(512, 4) else VB200_TC_LAUNCH(512, 3)
   } else if (BN == 256) VB200_TC_LAUNCH(256, 3) else VB200_TC_LAUNCH(128, 3)
 #undef VB200_TC_LAUNCH
   rc = check_launch("deform_conv2d_tc_kernel");
